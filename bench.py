@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- tracks/sec analysed (10 s @ 48 kHz) + k-NN queries/sec over 100 k embeddings.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the analysis hot path (PCM16 windows -> log-mel -> student CLAP encoder ->
@@ -19,6 +19,8 @@ Reported (ONE JSON line on rank 0):
   cpu_baseline   the oracle (CPU restatement of librosa + onnxruntime, reference libs are not
             installable) timed on this box's host cores on a bounded sample
 `--impl reference` times that CPU restatement as the arm itself (rank 0 only).
+`--dump-outputs DIR` writes what the last timed step computed to DIR/embeddings.npy (rank 0; inputs and weights are
+seeded, so two builds run with the same arguments can be compared output for output).
 """
 from __future__ import annotations
 
@@ -42,6 +44,7 @@ T_FRAMES = 1001
 METRIC = "tracks_per_sec_analysed_10s_48khz"
 UNIT = "tracks/s"
 WEIGHT_SEED = 0
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def _peaks():
@@ -206,6 +209,19 @@ def run_reference(args):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+
+
+def dump_embeddings(out_dir, emb):
+    """Writes the f32[n, dim] embeddings a caller of the timed path receives as out_dir/embeddings.npy.  Above
+    DUMP_LIMIT_BYTES a fixed seeded sample of rows is written instead, with their row numbers in embeddings_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    emb = np.ascontiguousarray(emb, dtype=np.float32)
+    max_rows = DUMP_LIMIT_BYTES // (emb.shape[1] * 4 + 8)
+    if len(emb) > max_rows:
+        rows = np.sort(np.random.default_rng(0).choice(len(emb), max_rows, replace=False))
+        emb = emb[rows]
+        np.save(os.path.join(out_dir, "embeddings_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "embeddings.npy"), emb)
 
 
 # ----------------------------------------------------------------------------------------------
@@ -412,6 +428,8 @@ def run_b200(args):
     barrier()
     ms = e0.elapsed_time(e1)
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_embeddings(args.dump_outputs, (gathered if world > 1 else out_dev).cpu().numpy())
     prof = _lib.profile_report()
     _lib.profile_enable(False)
     clocks = sampler.stop() if sampler else None
@@ -598,7 +616,11 @@ def main():
     ap.add_argument("--kmeans-rows", type=int, default=1_000_000)
     ap.add_argument("--profile-mode", action="store_true",
                     help="for runs under ncu: honour --warmup < 3; the printed numbers are NOT bench values")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the embeddings of the last timed step to DIR/embeddings.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,9 +1,9 @@
 #!/usr/bin/env python
 """Generate golden vectors by RUNNING THE REFERENCE'S OWN PYTHON CODE in the build container.
 
-    python tests/golden/make_golden.py          # needs /root/reference (not on the GPU box)
+    AUDIOMUSE_AI_SRC=<AudioMuse-AI checkout> python tests/golden/make_golden.py
 
-/root/reference is imported read-only.  Third-party modules that are not installed here
+The reference tree is imported read-only.  Third-party modules that are not installed here
 (librosa, onnxruntime, voyager, psycopg2, pydub, ...) are replaced by inert stubs so
 that the reference's *own* logic runs unmodified:
 
@@ -31,7 +31,7 @@ import types
 
 import numpy as np
 
-REF = "/root/reference"
+REF = os.environ.get("AUDIOMUSE_AI_SRC", "")
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -75,6 +75,8 @@ SEGMENT_CASE_LENGTHS = [1, 1000, 479_999, 480_000, 480_001, 700_000, 720_000, 72
 
 
 def main():
+    if not os.path.isdir(os.path.join(REF, "tasks")):
+        raise SystemExit("set AUDIOMUSE_AI_SRC to an AudioMuse-AI checkout")
     sys.path.insert(0, REF)
     os.environ.setdefault("TRANSFORMERS_NO_ADVISORY_WARNINGS", "1")
     import config  # the reference's config.py (pure env-var defaults)

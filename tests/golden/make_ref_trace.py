@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""Golden "call traces" of the reference's own query functions, for the GPU box (which has no /root/reference).
+"""Golden "call traces" of the reference's own query functions, so that the tests need no reference tree.
 
-    python tests/golden/make_ref_trace.py          # needs /root/reference; writes tests/golden/ref_trace.npz
+    AUDIOMUSE_AI_SRC=<AudioMuse-AI checkout> python tests/golden/make_ref_trace.py   # writes tests/golden/ref_trace.npz
 
 Runs, UNMODIFIED and over a recording brute-force index (tests/ref_harness.RecordingIndex = the reference tests'
 DummyVoyagerIndex contract with float64 ranking and lower-id ties),

@@ -1,10 +1,10 @@
-"""Test infrastructure: import the REFERENCE's own modules (read-only, from /root/reference) with inert stand-ins for
-the third-party packages that are not installed here (psycopg2, voyager, the Flask app helpers), so their functions
-run unmodified -- over a recording brute-force index when goldens are generated (tests/golden/make_ref_trace.py), or
-over audiomuse_ai_b200.voyager_compat when the shims themselves are under test (tests/test_reference_shims.py).
+"""Golden-generator infrastructure: import the REFERENCE's own modules (read-only, from the AudioMuse-AI checkout
+named by $AUDIOMUSE_AI_SRC) with inert stand-ins for the third-party packages that are not installed here (psycopg2,
+voyager, the Flask app helpers), so their functions run unmodified -- over a recording brute-force index
+(tests/golden/make_ref_trace.py), or over a recorder in front of audiomuse_ai_b200.voyager_compat
+(tests/golden/make_shim_trace.py).
 
-/root/reference does not exist on the GPU box: everything here is used by `-m "not gpu"` tests (which skip when the
-tree is absent) and by the golden generator, never by a `-m gpu` test.
+No test imports the reference: the tests replay what these generators stored under tests/golden/.
 """
 from __future__ import annotations
 
@@ -18,11 +18,11 @@ from typing import Dict, List, Optional
 
 import numpy as np
 
-REF = "/root/reference"
+REF = os.environ.get("AUDIOMUSE_AI_SRC", "")
 
 
 def available() -> bool:
-    return os.path.isdir(os.path.join(REF, "tasks"))
+    return bool(REF) and os.path.isdir(os.path.join(REF, "tasks"))
 
 
 # ------------------------------------------------------------------------------------------------ fake database
