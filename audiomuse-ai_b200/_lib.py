@@ -82,6 +82,17 @@ SIGNATURES = {
     "am_clap_embed_tracks_submit": (_i, [_vp, _P(MelCfg), _vp, _i, _vp, _i, _vp]),
     "am_clap_embed_tracks_collect": (_i, [_vp]),
     "am_clap_embed_tracks_dev": (_i, [_vp, _vp, _vp, _i, _vp, _i, _i, _vp, _vp]),
+    "am_musicnn_load": (_i, [C.c_char_p, _P(_vp)]),
+    "am_musicnn_load_mem": (_i, [_vp, _sz, _P(_vp)]),
+    "am_musicnn_describe_file": (_i, [C.c_char_p, C.c_char_p, _i]),
+    "am_musicnn_free": (None, [_vp]),
+    "am_musicnn_release_workspace": (_i, [_vp]),
+    "am_musicnn_dims": (_i, [_vp, _P(_i), _P(_i), _P(_i)]),
+    "am_musicnn_io_names": (_i, [_vp, C.c_char_p, C.c_char_p, _i]),
+    "am_musicnn_flops_per_patch": (C.c_double, [_vp, _i, _i, _P(C.c_double)]),
+    "am_musicnn_run": (_i, [_vp, _vp, _i, _i, _i, _vp]),
+    "am_musicnn_run_dev": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
+    "am_musicnn_analyze_tracks": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "am_knn_build": (_i, [_vp, _i64, _i, _i, _P(_vp)]),
     "am_knn_build_dev": (_i, [_vp, _i64, _i, _i, _vp, _P(_vp)]),
     "am_knn_free": (None, [_vp]),

@@ -47,10 +47,35 @@ def make_filter_by_distance(vm):
     return _filter_by_distance_b200
 
 
-def apply(clap=None, voyager_manager=None, clustering=None, allow_sklearn_fallback: bool = True) -> None:
-    """clap / voyager_manager / clustering: the reference's already imported tasks.* modules (pass only the ones to
-    patch).  allow_sklearn_fallback keeps the reference's contract that a failing GPU k-means silently falls back to
-    scikit-learn (tasks/clustering_gpu.py:130-148); this repository's own tests run with it off so a missing CUDA
+MUSICNN_MODEL_FILES = ("musicnn_embedding.onnx", "musicnn_prediction.onnx")
+
+
+class OrtProxy:
+    """Stands in for the `ort` (onnxruntime) module that tasks/analysis.py uses only for MusiCNN (:405-509, :763-841):
+    InferenceSession returns a B200 MusicnnSession for the two MusiCNN model files (config EMBEDDING_MODEL_PATH /
+    PREDICTION_MODEL_PATH) and the real session for anything else; every other attribute (get_available_providers,
+    capi.onnxruntime_pybind11_state.RuntimeException named by the reference's except clauses, ...) is the real
+    module's."""
+
+    def __init__(self, real):
+        self._real = real
+
+    def InferenceSession(self, path_or_bytes, *args, **kwargs):
+        if isinstance(path_or_bytes, (str, os.PathLike)) and os.path.basename(os.fspath(path_or_bytes)) in MUSICNN_MODEL_FILES:
+            from .musicnn import MusicnnSession
+
+            return MusicnnSession(os.fspath(path_or_bytes))
+        return self._real.InferenceSession(path_or_bytes, *args, **kwargs)
+
+    def __getattr__(self, name):
+        return getattr(self._real, name)
+
+
+def apply(clap=None, voyager_manager=None, clustering=None, allow_sklearn_fallback: bool = True, analysis=None) -> None:
+    """clap / voyager_manager / clustering / analysis: the reference's already imported tasks.* modules (pass only the
+    ones to patch).  analysis (tasks.analysis): its `ort` becomes an OrtProxy, so analyze_track's MusiCNN sessions run
+    on the B200 while its librosa tempo / chroma / RMS code stays as it is.  allow_sklearn_fallback keeps the
+    reference's contract that a failing GPU k-means silently falls back to scikit-learn (tasks/clustering_gpu.py:130-148); this repository's own tests run with it off so a missing CUDA
     library can never pass as the GPU path."""
     if clap is not None:
         from . import clap_analyzer as b200_clap
@@ -68,3 +93,5 @@ def apply(clap=None, voyager_manager=None, clustering=None, allow_sklearn_fallba
         clustering.check_gpu_available = b200_cg.check_gpu_available
         if allow_sklearn_fallback:
             os.environ.setdefault("B200_ALLOW_SKLEARN_FALLBACK", "1")
+    if analysis is not None and not isinstance(analysis.ort, OrtProxy):
+        analysis.ort = OrtProxy(analysis.ort)

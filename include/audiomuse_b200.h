@@ -190,6 +190,48 @@ AM_API int am_clap_embed_tracks_dev(am_model* m, const am_mel_plan* plan, const 
                              int n_samples, const int32_t* seg_offsets_dev, int n_tracks,
                              int n_segments, float* out_dev, void* stream);
 
+/* ------------------------------------------------------------------ MusiCNN tower
+ * Replaces the two onnxruntime sessions of tasks/analysis.py:405-509 (analyze_track):
+ *   EMBEDDING_MODEL_PATH  musicnn_embedding.onnx   'model/Placeholder:0' f32[n, 187, 96] -> 'model/dense/BiasAdd:0' f32[n, 200]
+ *   PREDICTION_MODEL_PATH musicnn_prediction.onnx  'serving_default_model_Placeholder:0' f32[n, 200]
+ *                                                  -> 'PartitionedCall:0' f32[n, 50] (raw logits)
+ * am_musicnn_load reads either file and lowers it (csrc/musicnn.cu: front-end branches conv -> ReLU -> BatchNorm ->
+ * frequency max, 7-tap mid-end with residuals, time max + mean pooling, BatchNorm / dense head; the prediction graph is
+ * a row program).  Any other node fails the load with its name and operator in am_last_error(). */
+typedef struct am_musicnn am_musicnn;
+AM_API int am_musicnn_load(const char* model_path, am_musicnn** out);
+AM_API int am_musicnn_load_mem(const void* blob, size_t nbytes, am_musicnn** out);
+/* host-only, needs no GPU: the lowered program as text (one line per branch / layer / head op); returns the size
+ * needed (NUL included) or a negative am_status */
+AM_API int am_musicnn_describe_file(const char* model_path, char* buf, int cap);
+AM_API void am_musicnn_free(am_musicnn* m);
+/* frees activations and staging buffers (weights stay): the cleanup step before the reference retries after an OOM
+ * (tasks/analysis.py:465-486) */
+AM_API int am_musicnn_release_workspace(am_musicnn* m);
+/* is_embedding: 1 for a patch graph, 0 for a row graph; in_dim: row width of a row graph (0 for patches) */
+AM_API int am_musicnn_dims(const am_musicnn* m, int* is_embedding, int* in_dim, int* out_dim);
+/* the graph's input and output tensor names (what onnxruntime's get_inputs() / get_outputs() report), NUL
+ * terminated, each buffer `cap` bytes; returns the capacity needed (nothing is written when cap is smaller) */
+AM_API int am_musicnn_io_names(const am_musicnn* m, char* in_name, char* out_name, int cap);
+/* 2 * multiply-accumulates of one [T, F] patch (embedding) or one row (prediction); *front_flops (optional) gets the
+ * front-end branches' share, counted from the graph's kernel shapes (no padding) */
+AM_API double am_musicnn_flops_per_patch(const am_musicnn* m, int T, int F, double* front_flops);
+/* run_inference (tasks/analysis.py:129-170) for either graph: embedding in f32[n, T, F] (T = 187, F = 96 in the
+ * reference), prediction in f32[n, in_dim] (pass T = in_dim, F = 1); out f32[n, out_dim] */
+AM_API int am_musicnn_run(am_musicnn* m, const float* in, int n, int T, int F, float* out);
+AM_API int am_musicnn_run_dev(am_musicnn* m, const float* in_dev, int n, int T, int F, float* out_dev, void* stream);
+/* Bulk analyze_track (tasks/analysis.py:368-544) for the MusiCNN outputs: 16 kHz mono PCM of n_tracks tracks,
+ * track t = pcm[offsets[t], offsets[t+1]) -> mel (n_fft 512, hop 256, 96 mels, center=False, log10(1 + 10000 x)) ->
+ * 187-frame patches -> embedding -> prediction; emb_out f32[n_tracks, 200] = mean of the patch embeddings (:544),
+ * moods_out f32[n_tracks, 50] = sigmoid(mean(sigmoid(logits))) (:521-522), n_patches i32[n_tracks].  A track too
+ * short for one patch gets n_patches 0 and zero rows (the reference returns no result for it, :378-381).
+ * pred / moods_out may be NULL.  Device memory: the PCM and the patches of ALL n_tracks are staged at once (4 bytes
+ * per sample + 72 KB per patch) on top of the model workspace (about 1.3 GB for the published widths: sub-batches of
+ * 512 patches, the first mid-end layer's 7 x 576-channel im2col is the largest part); callers bound n_tracks
+ * (musicnn.analyze_tracks sends at most 2^26 samples, about 70 minutes of audio, per call). */
+AM_API int am_musicnn_analyze_tracks(am_musicnn* emb, am_musicnn* pred, const float* pcm, const int64_t* offsets,
+                                     int n_tracks, float* emb_out, float* moods_out, int* n_patches);
+
 /* ------------------------------------------------------------------ K4: exact k-NN index
  * Replaces the voyager.Index object (voyager==2.1.0) used at tasks/voyager_manager.py:183,
  * 341-346,1397,1447,1580,1681 and tasks/clap_text_search.py:173,242,263,493.
