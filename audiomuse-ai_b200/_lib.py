@@ -33,6 +33,13 @@ class MelCfg(C.Structure):
                 ("fmin", C.c_float), ("fmax", C.c_float), ("transpose", C.c_int)]
 
 
+class TrackFeat(C.Structure):
+    """am_track_feat"""
+    _fields_ = [("tempo", C.c_double), ("tuning", C.c_double), ("energy", C.c_float), ("chroma_mean", C.c_float * 12),
+                ("period", C.c_int), ("key", C.c_int), ("is_major", C.c_int), ("n_frames", C.c_int),
+                ("n_pitches", C.c_int), ("tuning_counts", C.c_int * 100)]
+
+
 _vp, _i, _i64, _f, _u64, _sz = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_uint64, C.c_size_t
 _P = C.POINTER
 
@@ -93,6 +100,11 @@ SIGNATURES = {
     "am_musicnn_run": (_i, [_vp, _vp, _i, _i, _i, _vp]),
     "am_musicnn_run_dev": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
     "am_musicnn_analyze_tracks": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "am_features_create": (_i, [_P(_vp)]),
+    "am_features_free": (None, [_vp]),
+    "am_features_release_workspace": (_i, [_vp]),
+    "am_features_run": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
+    "am_features_run_dev": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "am_knn_build": (_i, [_vp, _i64, _i, _i, _P(_vp)]),
     "am_knn_build_dev": (_i, [_vp, _i64, _i, _i, _vp, _P(_vp)]),
     "am_knn_free": (None, [_vp]),

@@ -16,6 +16,7 @@
 //
 // Algorithmic traffic per 10 s window: 480000*2 B (PCM16) or *4 B (f32) in, 128*1001*4 B out.
 #include "common.cuh"
+#include "fft_reg.cuh"
 
 #include <cmath>
 
@@ -93,76 +94,6 @@ int build_filterbank(const am_mel_cfg& c, std::vector<float>& w /* [n_mels * bin
     }
   }
   return AM_OK;
-}
-
-// ---------------------------------------------------------------- device: 32-point FFT
-__device__ __forceinline__ float cos32(int i) {  // cos(2*pi*i/32), i in [0,16)
-  switch (i) {
-    case 0: return 1.0f;
-    case 1: return 0.98078528040323044913f;
-    case 2: return 0.92387953251128675613f;
-    case 3: return 0.83146961230254523708f;
-    case 4: return 0.70710678118654752440f;
-    case 5: return 0.55557023301960222474f;
-    case 6: return 0.38268343236508977173f;
-    case 7: return 0.19509032201612826785f;
-    case 8: return 0.0f;
-    case 9: return -0.19509032201612826785f;
-    case 10: return -0.38268343236508977173f;
-    case 11: return -0.55557023301960222474f;
-    case 12: return -0.70710678118654752440f;
-    case 13: return -0.83146961230254523708f;
-    case 14: return -0.92387953251128675613f;
-    default: return -0.98078528040323044913f;
-  }
-}
-// sin(2*pi*i/32) for i in [0,16): sin(x) = cos(x - pi/2) -> index i-8; cos is even.
-__device__ __forceinline__ float sin32i(int i) {
-  int j = i - 8;
-  if (j < 0) j = -j;
-  return cos32(j);
-}
-
-__host__ __device__ constexpr int rev5(int i) {
-  return ((i & 1) << 4) | ((i & 2) << 2) | (i & 4) | ((i & 8) >> 2) | ((i & 16) >> 4);
-}
-
-// In-place radix-2 decimation-in-frequency, forward (e^{-i...}).  Input natural order,
-// output bit-reversed: X[k] is left in element rev5(k).  Fully unrolled; all indices and
-// twiddles are compile-time, trivial twiddles cost no multiplies.
-__device__ __forceinline__ void fft32(float (&re)[32], float (&im)[32]) {
-#pragma unroll
-  for (int half = 16; half >= 1; half >>= 1) {
-#pragma unroll
-    for (int base = 0; base < 32; base += 2 * half) {
-#pragma unroll
-      for (int j = 0; j < half; ++j) {
-        const int a = base + j, b = a + half;
-        const float ar = re[a], ai = im[a], br = re[b], bi = im[b];
-        re[a] = ar + br;
-        im[a] = ai + bi;
-        const float dr = ar - br, di = ai - bi;
-        const int idx = j * (16 / half);  // twiddle W_32^idx = cos - i sin
-        if (idx == 0) {
-          re[b] = dr;
-          im[b] = di;
-        } else if (idx == 8) {  // * (-i)
-          re[b] = di;
-          im[b] = -dr;
-        } else if (idx == 4) {  // * (1 - i)/sqrt2
-          re[b] = (dr + di) * 0.70710678118654752440f;
-          im[b] = (di - dr) * 0.70710678118654752440f;
-        } else if (idx == 12) {  // * (-1 - i)/sqrt2
-          re[b] = (di - dr) * 0.70710678118654752440f;
-          im[b] = -(dr + di) * 0.70710678118654752440f;
-        } else {
-          const float c = cos32(idx), s = sin32i(idx);
-          re[b] = fmaf(dr, c, di * s);
-          im[b] = fmaf(di, c, -dr * s);
-        }
-      }
-    }
-  }
 }
 
 // ---------------------------------------------------------------- device: kernel
@@ -442,16 +373,8 @@ extern "C" int am_mel_plan_create(const am_mel_cfg* cfg, am_mel_plan** out) {
   // periodic Hann of the frame length; zero beyond it (frames shorter than 2048 are zero-padded transforms)
   std::vector<float> win(kNfft, 0.0f);
   for (int n = 0; n < cfg->n_fft; ++n) win[n] = (float)(0.5 - 0.5 * std::cos(2.0 * M_PI * n / cfg->n_fft));
-  std::vector<float2> ftw(32 * 32), ptw(kNc);
-  for (int k1 = 0; k1 < 32; ++k1)
-    for (int n2 = 0; n2 < 32; ++n2) {
-      const double a = 2.0 * M_PI * (double)(n2 * k1) / kNc;
-      ftw[k1 * 32 + n2] = make_float2((float)std::cos(a), (float)-std::sin(a));
-    }
-  for (int k = 0; k < kNc; ++k) {
-    const double a = 2.0 * M_PI * k / kNfft;
-    ptw[k] = make_float2((float)std::cos(a), (float)-std::sin(a));
-  }
+  std::vector<float2> ftw, ptw;
+  fill_fft_twiddles(ftw, ptw);
   auto* plan = new am_mel_plan();
   plan->cfg = *cfg;
   plan->max_bin = max_bin;

@@ -71,12 +71,87 @@ class OrtProxy:
         return getattr(self._real, name)
 
 
-def apply(clap=None, voyager_manager=None, clustering=None, allow_sklearn_fallback: bool = True, analysis=None) -> None:
+def make_analyze_track(analysis):
+    """analyze_track (tasks/analysis.py:324-573) with everything after decoding on the B200: the tempo / energy /
+    key / scale features (track_features) and the MusiCNN embedding + moods (musicnn.analyze_tracks).  Same signature
+    and the same 2- or 4-tuples; an empty, silent, too-short or failed track gives the None tuple, as upstream.
+    Decoding stays the reference's own: analysis.robust_load_audio_with_fallback, looked up at call time.
+    MusiCNN sessions come from onnx_sessions when they are B200 MusicnnSessions, else from model_paths (loaded once
+    per path).  On B200OutOfMemory the workspaces are released and the track is retried once."""
+    import logging
+
+    import numpy as np
+
+    from . import _lib, musicnn, track_features as tfm
+
+    log = logging.getLogger(__name__)
+    state = {"features": None, "sessions": {}}
+
+    def _sessions(model_paths, onnx_sessions):
+        if onnx_sessions is not None and all(isinstance(onnx_sessions.get(k), musicnn.MusicnnSession)
+                                             for k in ("embedding", "prediction")):
+            return onnx_sessions["embedding"], onnx_sessions["prediction"]
+        out = []
+        for k in ("embedding", "prediction"):
+            path = os.fspath(model_paths[k])
+            if path not in state["sessions"]:
+                state["sessions"][path] = musicnn.MusicnnSession(path)
+            out.append(state["sessions"][path])
+        return tuple(out)
+
+    def _run(audio, emb, pred):
+        if state["features"] is None:
+            state["features"] = tfm.FeatureSession()
+        feats = tfm.track_features([audio], session=state["features"])[0]
+        tower = musicnn.analyze_tracks([audio], emb, pred)[0]
+        return feats, tower
+
+    def analyze_track(file_path, mood_labels_list, model_paths, onnx_sessions=None, return_audio=False):
+        none = (None, None, None, None) if return_audio else (None, None)
+        audio, sr = analysis.robust_load_audio_with_fallback(file_path, target_sr=16000)
+        if audio is None or audio.size == 0 or not np.any(audio):
+            log.warning("Could not load a valid audio signal for %s. Skipping track.", os.path.basename(file_path))
+            return none
+        audio = np.ascontiguousarray(audio, dtype=np.float32).reshape(-1)
+        try:
+            emb, pred = _sessions(model_paths, onnx_sessions)
+            try:
+                feats, tower = _run(audio, emb, pred)
+            except _lib.B200OutOfMemory:
+                log.warning("B200 out of memory for %s: releasing workspaces and retrying once",
+                            os.path.basename(file_path))
+                for s in (state["features"], emb, pred):
+                    if s is not None:
+                        s.release_workspace()
+                feats, tower = _run(audio, emb, pred)
+        except _lib.B200Error as e:
+            log.error("B200 analysis failed for %s: %s", os.path.basename(file_path), e)
+            return none
+        if tower is None or feats is None:
+            log.warning("Track too short to create spectrogram patches: %s", os.path.basename(file_path))
+            return none
+        embedding, moods, _ = tower
+        result = {"tempo": feats["tempo"], "key": feats["key"], "scale": feats["scale"],
+                  "moods": {label: float(v) for label, v in zip(mood_labels_list, moods)},
+                  "energy": feats["energy"]}
+        embedding = np.asarray(embedding, dtype=np.float32)
+        return (result, embedding, audio, sr) if return_audio else (result, embedding)
+
+    analyze_track._b200 = True
+    return analyze_track
+
+
+def apply(clap=None, voyager_manager=None, clustering=None, allow_sklearn_fallback: bool = True, analysis=None,
+          analyze_track: bool = False) -> None:
     """clap / voyager_manager / clustering / analysis: the reference's already imported tasks.* modules (pass only the
     ones to patch).  analysis (tasks.analysis): its `ort` becomes an OrtProxy, so analyze_track's MusiCNN sessions run
-    on the B200 while its librosa tempo / chroma / RMS code stays as it is.  allow_sklearn_fallback keeps the
+    on the B200.  With analyze_track=True, analysis.analyze_track itself is replaced by make_analyze_track(analysis)
+    (analyze_album_task resolves that module global at call time), so its librosa tempo / energy / chroma code runs
+    on the B200 too; with the default False that code stays as it is.  allow_sklearn_fallback keeps the
     reference's contract that a failing GPU k-means silently falls back to scikit-learn (tasks/clustering_gpu.py:130-148); this repository's own tests run with it off so a missing CUDA
     library can never pass as the GPU path."""
+    if analyze_track and analysis is None:
+        raise ValueError("apply(analyze_track=True) needs the analysis module")
     if clap is not None:
         from . import clap_analyzer as b200_clap
 
@@ -95,3 +170,5 @@ def apply(clap=None, voyager_manager=None, clustering=None, allow_sklearn_fallba
             os.environ.setdefault("B200_ALLOW_SKLEARN_FALLBACK", "1")
     if analysis is not None and not isinstance(analysis.ort, OrtProxy):
         analysis.ort = OrtProxy(analysis.ort)
+    if analyze_track and not getattr(analysis.analyze_track, "_b200", False):
+        analysis.analyze_track = make_analyze_track(analysis)

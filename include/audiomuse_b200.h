@@ -232,6 +232,41 @@ AM_API int am_musicnn_run_dev(am_musicnn* m, const float* in_dev, int n, int T, 
 AM_API int am_musicnn_analyze_tracks(am_musicnn* emb, am_musicnn* pred, const float* pcm, const int64_t* offsets,
                                      int n_tracks, float* emb_out, float* moods_out, int* n_patches);
 
+/* ------------------------------------------------------------------ Track features
+ * The librosa part of analyze_track (tasks/analysis.py:344-365) for 16 kHz mono tracks, track t =
+ * pcm[offsets[t], offsets[t+1]) (csrc/track_features.cu; oracle/track_features.py restates it):
+ *   tempo   beat_track's tempo: 60 * 16000 / (512 * period), 0 when the onset envelope is all zero
+ *   energy  np.mean(librosa.feature.rms(y))
+ *   tuning  estimate_tuning of the power spectrogram; chroma_mean = mean over frames of chroma_stft(tuning)
+ *   key     index into C, C#, ..., B of the key / scale block; is_major is always 0 there (the minor profile is the
+ *           major one rolled by 3, so `major_max > minor_max` never holds)
+ * tuning_counts / n_pitches: the tuning histogram over linspace(-0.5, 0.5, 101) and the pitches it counts.
+ * An empty track gets n_frames 0 and zeros.  Device memory: about 13 bytes per sample of the call (8 of them the
+ * power spectrogram); callers bound a call's size (track_features.track_features sends at most 2^26 samples). */
+typedef struct am_track_feat {
+  double tempo;
+  double tuning;
+  float energy;
+  float chroma_mean[12];
+  int period;
+  int key;
+  int is_major;
+  int n_frames;
+  int n_pitches;
+  int tuning_counts[100];
+} am_track_feat;
+typedef struct am_features am_features;
+AM_API int am_features_create(am_features** out);
+AM_API void am_features_free(am_features* h);
+/* frees every per-call buffer (the tables stay) */
+AM_API int am_features_release_workspace(am_features* h);
+/* tempogram (nullable): f32[n_tracks, 250], the per-lag mean of each track's normalised tempogram */
+AM_API int am_features_run(am_features* h, const float* pcm, const int64_t* offsets, int n_tracks,
+                           am_track_feat* out, float* tempogram);
+/* the same with device-resident PCM (offsets, out and tempogram stay on the host), ordered on `stream` */
+AM_API int am_features_run_dev(am_features* h, const float* pcm_dev, const int64_t* offsets, int n_tracks,
+                               am_track_feat* out, float* tempogram, void* stream);
+
 /* ------------------------------------------------------------------ K4: exact k-NN index
  * Replaces the voyager.Index object (voyager==2.1.0) used at tasks/voyager_manager.py:183,
  * 341-346,1397,1447,1580,1681 and tasks/clap_text_search.py:173,242,263,493.
